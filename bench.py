@@ -23,6 +23,9 @@ dataset has N x that, sharded by kb_shard_of(subject, N); a subject-star join ne
              strong = the 100 M-triple store of BASELINE configs[2] split over the N GPUs (strong scaling)
   cfg2_10M   (N = 1) the same query on BASELINE configs[1]'s own 10 M-triple store: the size the CPU arm runs
   cpu_baseline / --impl reference: the oracle's restatement of the reference's own algorithm, timed on the host cores
+
+--dump-outputs DIR writes the binding rows the headline's last timed step returned (see write_outputs), so that two builds of the
+project can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -34,6 +37,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -64,7 +68,13 @@ def parse_args():
                     "step; off by default: the one 8-rank run with it on also showed a 3x slower host side of the resident step)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-index", action="store_true", help="headline on the store-scanning path (no predicate-partitioned index)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="write the rows the headline's last timed step returned to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config or args.impl == "reference"):
+        ap.error("--dump-outputs writes the headline's result: not with --config or --impl reference")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -276,8 +286,9 @@ def workload_name(args):
     return f"employee shape, {args.employees} employees = {6 * args.employees} triples per GPU, {q}"
 
 
-def run_pipelined(plan, steps):
-    """K prepared queries back to back: submit, and collect the query submitted ring-1 steps earlier. Returns the last row count."""
+def run_pipelined(plan, steps, keep=None):
+    """K prepared queries back to back: submit, and collect the query submitted ring-1 steps earlier. Returns the last row count.
+    With a list `keep`, the last query's rows are appended to it (a Relation view of the plan's ring slot)."""
     depth = max(1, plan.ring - 1)
     inflight = []
     rows = 0
@@ -286,8 +297,34 @@ def run_pipelined(plan, steps):
         if len(inflight) > depth:
             rows = plan.collect(inflight.pop(0))
     while inflight:
-        rows = plan.collect(inflight.pop(0))
+        if keep is not None and len(inflight) == 1:
+            keep.append(plan.collect_rows(inflight.pop(0)))
+            rows = keep[-1].n_rows
+        else:
+            rows = plan.collect(inflight.pop(0))
     return rows
+
+
+DUMP_BYTES = 60_000_000  # --dump-outputs: at most this many bytes of rows in all (over all ranks)
+
+
+def write_outputs(out_dir, rel, rank, world):
+    """--dump-outputs: the rows `rel` holds, columns in ascending slot order, as DIR/bindings.npy (float64: u32 ids are exact in it),
+    sorted lexicographically so that two builds compare row for row whatever order their kernels emit them in. Above the size bound a
+    fixed seeded sample of the sorted rows is written; DIR/bindings_index.npy holds the positions of the written rows among the
+    sorted ones, DIR/row_count.npy the number of rows. With several ranks every rank writes its own rows, suffixed _rank<r>."""
+    from kolibrie_b200 import datagen
+
+    rows = datagen.canonical_rows(rel.to_numpy(sorted(rel.slots)))
+    cap = DUMP_BYTES // (8 * (rows.shape[1] + 1) * world)
+    idx = np.arange(len(rows))
+    if len(rows) > cap:
+        idx = np.sort(np.random.default_rng(0).choice(len(rows), size=cap, replace=False))
+    sfx = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"bindings{sfx}.npy"), rows[idx].astype(np.float64))
+    np.save(os.path.join(out_dir, f"bindings_index{sfx}.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, f"row_count{sfx}.npy"), np.array([len(rows)], dtype=np.float64))
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -365,10 +402,13 @@ def main():
     js, pats, filt = datagen.employee_queries(d)[args.query]
     plan = None if args.no_index else ctx.prepare_star_join(js, pats, filt, ring=args.ring)
 
-    def step_sync():
+    def step_sync(keep=None):
         r = ctx.star_join(js, pats, filt)
         rows = r.n_rows
-        r.free()
+        if keep is not None:
+            keep.append(r)
+        else:
+            r.free()
         return rows
 
     # rank 0 samples all GPUs of the job through warm-up, the timed region and the e2e leg (all of it is load)
@@ -388,11 +428,18 @@ def main():
         barrier()
         return rows, t1 - t0, ctx.get_stats(reset=True)
 
-    sync_loop = lambda k: [step_sync() for _ in range(k)][-1]
-    head_fn = (lambda k: run_pipelined(plan, k)) if plan else sync_loop
+    def sync_loop(k, keep=None):
+        """k synchronous steps; with a list `keep`, the last step's rows are appended to it"""
+        return [step_sync(keep if i == k - 1 else None) for i in range(k)][-1]
+
+    head_fn = (lambda k, keep=None: run_pipelined(plan, k, keep)) if plan else sync_loop
     head_fn(W)
     ctx.set_timing(True)
-    rows_step, dt, st = timed(head_fn, K)
+    last = [] if args.dump_outputs else None
+    rows_step, dt, st = timed(lambda k: head_fn(k, last), K)
+    if last:
+        write_outputs(args.dump_outputs, last[0], rank, world)
+        last[0].free()
     # the same K steps through the synchronous operator (one host round trip per step)
     sync_leg = None
     def timed_best(fn, k, reps=3):
@@ -647,7 +694,7 @@ def other_configs(args, ctx, c, datagen, torch, peak, which=("cfg3", "cfg4", "cf
     from tests import oracle_api as O
 
     out = {}
-    K = max(5, min(args.steps, 20))
+    K = args.steps
 
     def frac(bytes_, ms):
         return (bytes_ / (ms * 1e-3) / 1e9) / peak if ms > 0 else None

@@ -105,22 +105,17 @@ def test_ctypes_signatures_match_the_header():
 
 def test_legacy_header_is_the_signature_kolibrie_binds():
     """include/cudajoin.h against the definition it replaces (kolibrie/src/cuda/cuda_join.cu:48-56) and the Rust declaration that calls it
-    (cuda_join.rs:14-26): parameter for parameter. Needs the reference checkout, which only the build container has."""
-    ref_cu = "/root/reference/kolibrie/src/cuda/cuda_join.cu"
-    ref_rs = "/root/reference/kolibrie/src/cuda/cuda_join.rs"
-    if not (os.path.exists(ref_cu) and os.path.exists(ref_rs)):
-        pytest.skip("no reference checkout on this machine")
+    (cuda_join.rs:14-26): parameter for parameter. Both parameter lists are stored in tests/golden/reference/cuda_join_signature.json."""
+    import json
 
-    def params(text, opener):
-        body = text[text.index(opener) + len(opener):]
-        body = body[: body.index(")")]
-        body = re.sub(r"/\*.*?\*/|//[^\n]*", " ", body, flags=re.S)
-        return [" ".join(x.split()) for x in body.split(",") if x.strip()]
+    from tests.golden.reference.make_reference_golden import c_params
 
-    ours = params(open(os.path.join(ROOT, "include", "cudajoin.h")).read(), "void perform_hash_join_cuda(")
-    theirs = params(open(ref_cu).read(), "void perform_hash_join_cuda(")
+    with open(os.path.join(ROOT, "tests", "golden", "reference", "cuda_join_signature.json")) as f:
+        ref = json.load(f)
+    ours = c_params(open(os.path.join(ROOT, "include", "cudajoin.h")).read(), "void perform_hash_join_cuda(")
+    theirs = ref["cuda_join.cu"]
     assert ours == theirs, (ours, theirs)
-    rust = params(open(ref_rs).read(), "pub fn perform_hash_join_cuda(")
+    rust = ref["cuda_join.rs"]
     assert [x.split(":")[0].strip() for x in rust] == [re.findall(r"\w+", x)[-1] for x in ours]
     depth = lambda t: t.count("*")
     assert [depth(x.split(":")[1]) for x in rust] == [depth(x) for x in ours], "pointer depth per parameter as Rust passes it"

@@ -353,18 +353,19 @@ def test_legacy_ffi_symbol(ctx):
 
 
 def test_legacy_vs_reference_cuda_stub():
-    """oracle/_ref/libcudajoin_ref.so is the reference's OWN cuda_join.cu compiled for sm_100a. Inside the range its clamped grid
-    covers, our symbol must return the same index SET (the reference's order is atomicAdd arrival order)."""
+    """The reference's OWN cuda_join.cu compiled for sm_100a, run on a B200: the index SET it returned for a seeded input inside the
+    range its clamped grid covers is stored in tests/golden/reference/cuda_stub_salary.npz (sorted: the reference's order is atomicAdd
+    arrival order). Our symbol must return that set for the same input."""
     import os
 
-    ref = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libcudajoin_ref.so")
-    if not os.path.exists(ref):
-        pytest.skip("reference CUDA stub not built")
-    d = datagen.employee_dataset(30000)  # 180 000 triples < 148 SMs * 2048 threads
-    pred = d.ids["ds:annual_salary"]
-    theirs = c.legacy_hash_join_cuda(d.s, d.p, d.o, pred, libpath=ref)
-    ours = c.legacy_hash_join_cuda(d.s, d.p, d.o, pred)
-    assert np.array_equal(np.sort(theirs), ours)
+    from tests.golden.reference.make_reference_golden import stub_input
+
+    golden = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "cuda_stub_salary.npz"))
+    s, p, o, pred, digest = stub_input()
+    assert digest == str(golden["input_sha256"]) and pred == int(golden["predicate"]), "the seeded input differs from the stored one"
+    theirs = golden["indices"]
+    ours = c.legacy_hash_join_cuda(s, p, o, pred)
+    assert len(theirs) == 30000 and np.array_equal(theirs, ours)
 
 
 def test_star_join_host_one_shot(ctx, emp):
